@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native LZ4 block codec (see BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 The metric is "GB/s uncompressed (encode+decode) on batched 64 KiB blocks": a STEP is one
@@ -142,6 +142,27 @@ def gen_blocks(n_blocks: int, match_proba: float, first_block: int, out: np.ndar
     with ThreadPoolExecutor(max_workers=min(64, os.cpu_count() or 1)) as ex:
         list(ex.map(run, jobs))
     return buf
+
+
+DUMP_BLOCKS = 64                # --dump-outputs: blocks whose bytes are written (2 x 16 MiB as float32)
+
+
+def dump_sample(n_blocks: int) -> np.ndarray:
+    """The fixed, seeded sample of block indices whose bytes --dump-outputs writes."""
+    return np.sort(np.random.default_rng(SEED).choice(n_blocks, min(DUMP_BLOCKS, n_blocks), replace=False))
+
+
+def write_outputs(out_dir: str, idx: np.ndarray, enc_len: np.ndarray, enc_slots: np.ndarray,
+                  dec_len: np.ndarray, dec_blocks: np.ndarray) -> None:
+    """--dump-outputs: what the last timed step returned to its caller, as <out_dir>/<name>.npy -- the
+    encode and decode lengths of every block (float64) and, for the blocks `idx`, the compressed bytes
+    (one compressBound slot per block, zero past the block's length) and the decoded bytes (float32)."""
+    os.makedirs(out_dir, exist_ok=True)
+    enc_slots = np.where(np.arange(BOUND)[None, :] < enc_len[idx][:, None], enc_slots, 0)
+    for name, a, dt in (("sample_blocks", idx, np.float64), ("encode_lengths", enc_len, np.float64),
+                        ("encode_bytes", enc_slots, np.float32), ("decode_lengths", dec_len, np.float64),
+                        ("decode_bytes", dec_blocks, np.float32)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(dt))
 
 
 def bind_to_gpu_numa_node(index: int) -> str:
@@ -294,6 +315,10 @@ def run_reference_arm(args) -> None:
     nb = args.blocks
     w = CpuWorkload(nb, 0, threads)
     te, td = w.time_steps(args.warmup, args.steps)
+    if args.dump_outputs:
+        idx = dump_sample(nb)
+        write_outputs(args.dump_outputs, idx, w.enc_len, w.slots.reshape(nb, BOUND)[idx], w.out_len,
+                      w.out.reshape(nb, BLOCK)[idx])
     ok = w.verify()
     r = cpu_numbers(w, te, td)
     t = sum(te) + sum(td)
@@ -473,6 +498,11 @@ def run_ours(args) -> None:
     torch.cuda.synchronize()
     clocks = sampler.stop() if rank == 0 else None
     paths = B.decode_stats(local, reset=True)
+    if args.dump_outputs and rank == 0:              # rank 0's slice: blocks [0, nb) of the global list
+        idx = dump_sample(nb)
+        d_idx = torch.from_numpy(idx).to(dev)
+        write_outputs(args.dump_outputs, idx, enc_len.cpu().numpy(), slots.view(nb, BOUND)[d_idx].cpu().numpy(),
+                      out_len.cpu().numpy(), out.view(nb, BLOCK)[d_idx].cpu().numpy())
     enc_ms = [e[0].elapsed_time(e[1]) for e in evs]
     dec_ms = [e[1].elapsed_time(e[2]) for e in evs]
     total_s = reduce_max_seconds(evs[0][0].elapsed_time(evs[-1][2]) / 1e3)
@@ -691,7 +721,12 @@ def main():
                          "runs on rank 0 whenever more than one GPU is visible)")
     ap.add_argument("--lib", default=None, help="development only: another build of libk4lz4.so (A/B runs of kernel variants)")
     ap.add_argument("--no-aux", action="store_true", help="development only: skip the aux legs (pickler, all-devices call)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                         "(lengths of every block, bytes of a fixed sample of blocks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

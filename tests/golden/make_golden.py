@@ -1,9 +1,10 @@
-"""Generates the committed golden fixtures.  Run in the build container (needs /root/reference):
+"""Generates the committed golden fixtures from a checkout of the reference (K4os.Compression.LZ4, whose
+orig/ holds the upstream lz4 C sources):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 1. issue64_block0.{lz4,bin}: the reference's own golden DECODE vector -- block #0 of
-   /root/reference/assets/issue64/input.dat (a "bv41" container: 12-byte header at byte 20,
+   <reference>/assets/issue64/input.dat (a "bv41" container: 12-byte header at byte 20,
    14 505 compressed bytes -> 65 536 bytes == output.dat[0:65536]); exercised by the
    reference's Issue64.cs:16-55.  issue64_block1.{lz4,bin}: block #1 of the same file (366 -> 3 034
    bytes), which only decodes with block #0's output as external dictionary.
@@ -13,14 +14,21 @@
    produced -- like the reference's own rows (playground/SharedSources/app.cpp:94-97) -- by the
    upstream C engine orig/lib/lz4.c compiled as-is (oracle/_ref/libk4ref.so), including
    limited-output capacities and the expected return codes.
+3. ref_engine.npz: that engine's results (return value, CRC-32 of the output) on every case set of
+   tests/inputs.py -- encode, decode of malformed streams, dictionary and partial decode, XXH32, the
+   data generator, and upstream lz4frame.c's frames -- which the tests compare the oracle and the
+   frame writer with.  Needs libk4lz4.so built (the synth inputs), no GPU.
 """
 import base64
 import hashlib
 import json
 import os
 import struct
+import subprocess
 import sys
 import zlib
+
+import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
@@ -29,15 +37,13 @@ sys.path.insert(0, ROOT)
 import oracle  # noqa: E402
 from tests import inputs  # noqa: E402
 
-REF = "/root/reference"
 
-
-def main():
-    oracle.build()
+def main(ref_dir):
+    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "REF=" + os.path.abspath(ref_dir)], check=True)
     R = oracle.Ref()
     # 1. issue64
-    blob = open(os.path.join(REF, "assets/issue64/input.dat"), "rb").read()
-    expect = open(os.path.join(REF, "assets/issue64/output.dat"), "rb").read()
+    blob = open(os.path.join(ref_dir, "assets/issue64/input.dat"), "rb").read()
+    expect = open(os.path.join(ref_dir, "assets/issue64/output.dat"), "rb").read()
     assert blob[20:24] == b"bv41"
     usize, csize = struct.unpack("<II", blob[24:32])
     comp = blob[32:32 + csize]
@@ -79,6 +85,22 @@ def main():
               open(os.path.join(HERE, "encode_rows.json"), "w"), indent=0)
     print(len(rows), "encode rows; issue64 ok")
 
+    # 3. the reference engine's results on the case sets of tests/inputs.py
+    P = oracle.Port()
+    sets = {}
+    for name, rows_of in inputs.ENGINE_SETS.items():
+        sets[name] = np.array(rows_of(P, R)[1], dtype=np.int64)
+
+    def upstream_frame(d, bc, cc):
+        f = R.frame_compress(d, bc, cc)
+        assert R.frame_decompress(f, len(d) + 16) == d
+        return f
+    sets["frame"] = np.array(inputs.frame_rows(P, upstream_frame)[1], dtype=np.int64)
+    np.savez_compressed(inputs.REF_RESULTS, **sets)
+    print({k: len(v) for k, v in sets.items()}, "reference results")
+
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

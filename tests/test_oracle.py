@@ -3,8 +3,8 @@
 * against the reference's own golden decode vector (assets/issue64 via Issue64.cs:16-55),
 * against committed known-answer encode rows made by the reference's upstream C engine
   (tests/golden/make_golden.py; style of ChecksumBlockTests.cs:185-216),
-* differentially against that engine itself (oracle/_ref) where it is present, including
-  malformed streams, and
+* differentially against that engine's recorded results (tests/golden/ref_engine.npz, made by
+  tests/golden/make_golden.py from the engine itself), including malformed streams, and
 * the reference's roundtrip / boundary tests (BlockRoundtripTests.cs:44-125) and pickler
   tests (PicklingTests.cs:11-172) restated on the oracle.
 """
@@ -51,32 +51,11 @@ def test_golden_encode_rows(port):
 
 
 def test_port_equals_reference_engine(port, ref):
-    for name, data in inputs.corpus(sizes=inputs.THRESHOLD_SIZES + inputs.BIG_SIZES):
-        a, b = ref.encode(data), port.encode(data)
-        assert a == b, name
-        n = len(data)
-        for cap in {n, n + 1, n - 1, 2 * n, max(n - 13, 0)}:
-            x, y = ref.decode(a[1], cap), port.decode(a[1], cap)
-            assert x[0] == y[0], (name, cap)
-            if x[0] > 0:
-                assert x[1] == y[1]
+    ref.check("corpus", *inputs.corpus_rows(port, port))
 
 
 def test_malformed_decode_matches_reference_engine(port, ref):
-    rng = np.random.default_rng(7)
-    checked = 0
-    for it in range(6000):
-        n = int(rng.choice([20, 50, 100, 300, 1000, 5000]))
-        kind = ["text2", "lowent", "runs", "random", "lorem"][it % 5]
-        data = inputs.gen(kind, n, it)
-        c = inputs.mutate(port.encode(data)[1], rng)
-        cap = int(rng.choice([n, n, n + 5, n - 1, 2 * n, n + 64, 0, 1]))
-        a, b = ref.decode(c, cap), port.decode(c, cap)
-        assert a[0] == b[0], (it, kind, n, cap)
-        if a[0] > 0 and not inputs.uses_zero_offset(c):   # offset-0 content is unspecified
-            assert a[1] == b[1]
-        checked += 1
-    assert checked == 6000
+    ref.check("malformed", *inputs.malformed_rows(port, port))      # offset-0 content is unspecified
 
 
 def test_enforce32_differs_only_for_large_inputs(port):
@@ -155,11 +134,7 @@ def test_pickler_restatement(port):
 
 def test_datagen_port_matches_reference_generator(port, ref):
     """oracle/datagen_port.c == the reference's own orig/programs/datagen.c (SURVEY 8(d) workload)."""
-    for size, mp, lp, seed in [(1 << 20, 0.63, 0.0, 1234), (1 << 20, 0.55, 0.0, 1234), (300001, 0.3, 0.0, 7),
-                               (65536, 0.9, 0.25, 99), (1, 0.63, 0.0, 1), (0, 0.63, 0.0, 1)]:
-        a = port.datagen(size, mp, lp, seed)
-        b = ref.datagen(size, mp, lp, seed)
-        assert np.array_equal(a, b), (size, mp, lp, seed)
+    ref.check("datagen", *inputs.datagen_rows(port, port))
     # the configs[1] / configs[2] ratios the survey probed (0.502 / 0.572 at 64 KiB blocks)
     for mp, lo, hi in [(0.63, 0.49, 0.515), (0.55, 0.56, 0.585)]:
         raw = port.datagen(64 * 65536, mp, 0.0, 1234)
@@ -167,16 +142,15 @@ def test_datagen_port_matches_reference_generator(port, ref):
         assert lo < tot / raw.size < hi, (mp, tot / raw.size)
 
 
-def test_issue64_block1_needs_block0_as_dictionary(port, ref):
+def test_issue64_block1_needs_block0_as_dictionary(port):
     """The reference's second golden vector (Issue64.cs:39-49): 366 -> 3 034 bytes with block #0's
     output as external dictionary (LZ4Codec.cs:144-157, LL64.dec.cs:338-378,523-546)."""
     comp = open(os.path.join(G, "issue64_block1.lz4"), "rb").read()
     expect = open(os.path.join(G, "issue64_block1.bin"), "rb").read()
     dic = open(os.path.join(G, "issue64_block0.bin"), "rb").read()
-    for eng in (port, ref):
-        assert eng.decode_dict(comp, 3034, dic) == (3034, expect)
-        assert eng.decode_dict(comp, 5000, dic) == (3034, expect)
-        assert eng.decode_dict(comp, 3033, dic)[0] == -1
+    assert port.decode_dict(comp, 3034, dic) == (3034, expect)
+    assert port.decode_dict(comp, 5000, dic) == (3034, expect)
+    assert port.decode_dict(comp, 3033, dic)[0] == -1
     assert port.decode(comp, 3034)[0] == -1          # without the dictionary the offsets fall outside
     assert port.decode_dict(comp, 3034, dic[1000:])[1] != expect or True
 
@@ -185,22 +159,7 @@ def test_dictionary_decode_matches_reference_engine(port, ref):
     """Blocks whose matches reach into an external dictionary: build them by compressing
     dict+data as one buffer and cutting the stream is not possible with the block API, so
     mutate offsets of ordinary streams instead -- every return code and every byte must agree."""
-    rng = np.random.default_rng(5)
-    for it in range(3000):
-        n = int(rng.choice([40, 200, 1000, 5000]))
-        kind = ["text2", "lowent", "runs", "lorem", "random"][it % 5]
-        data = inputs.gen(kind, n, it)
-        c = bytearray(port.encode(data)[1])
-        dic = inputs.gen("text2", int(rng.choice([1, 7, 64, 300, 4096, 70000])), it + 1)
-        if it % 3 and len(c) > 8:       # enlarge some offsets so that matches start inside the dictionary
-            for _ in range(3):
-                i = int(rng.integers(1, len(c) - 2))
-                c[i] = int(rng.integers(0, 256))
-        cap = int(rng.choice([n, n + 9, n - 1, 2 * n]))
-        a, b = ref.decode_dict(bytes(c), cap, dic), port.decode_dict(bytes(c), cap, dic)
-        assert a[0] == b[0], (it, kind, n, cap)
-        if a[0] > 0 and not inputs.uses_zero_offset(bytes(c)):
-            assert a[1] == b[1], (it, kind)
+    ref.check("dictionary", *inputs.dictionary_rows(port, port))
 
 
 def test_partial_decode_matches_reference_engine(port, ref):
@@ -208,19 +167,11 @@ def test_partial_decode_matches_reference_engine(port, ref):
     streams the restatement of LL64.dec.cs (lz4 1.9.2 text) and the upstream engine (1.9.3-dev,
     whose partial decoder was reworked) agree byte for byte; on malformed streams their accept
     decisions differ, and the C# text -- the restatement -- is the authority there."""
-    rng = np.random.default_rng(9)
-    for it in range(3000):
-        n = int(rng.choice([30, 100, 1000, 5000, 70000]))
-        kind = ["text2", "lowent", "runs", "lorem", "random"][it % 5]
-        data = inputs.gen(kind, n, it)
-        c = port.encode(data)[1]
-        target = int(rng.choice([0, 1, 5, 12, 13, n // 3, n // 2, n - 1, n, n + 1, 2 * n]))
-        a, b = ref.partial_decode(c, target), port.partial_decode(c, target)
-        assert a == b, (it, kind, n, target)
-        want = min(target, n)
-        assert b == ((want, data[:want]) if want > 0 else (-1, b""))
-        m = inputs.mutate(c, rng)                      # malformed: bounded, never past the target
-        r, out = port.partial_decode(m, target)
+    ref.check("partial", *inputs.partial_rows(port, port))
+    for _, data, c, target, m in inputs.partial_decode_cases(port):
+        want = min(target, len(data))
+        assert port.partial_decode(c, target) == ((want, data[:want]) if want > 0 else (-1, b""))
+        r, out = port.partial_decode(m, target)        # malformed: bounded, never past the target
         assert r == -1 or 0 < r <= max(target, 0)
 
 
@@ -234,8 +185,4 @@ def test_partial_decode_reference_cases(port):
 
 def test_xxh32_restatement_matches_upstream(port, ref):
     """oracle XXH32 == orig/lib/xxhash.c (the checksum of the LZ4 Frame container)."""
-    rng = np.random.default_rng(2)
-    for n in [0, 1, 3, 4, 15, 16, 17, 31, 32, 33, 100, 65536, 100001]:
-        a = rng.integers(0, 256, n, dtype=np.uint8)
-        for seed in (0, 1, 0xDEADBEEF):
-            assert port.xxh32(a, seed) == ref.xxh32(a, seed), (n, seed)
+    ref.check("xxh32", *inputs.xxh32_rows(port, port))

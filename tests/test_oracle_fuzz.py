@@ -1,46 +1,14 @@
-"""Property-based differential pinning of the oracle restatement against the reference's upstream C
-engine (oracle/_ref), CPU only: arbitrary byte strings as INPUT of Encode (identical bytes and
-return codes for every capacity class) and as COMPRESSED STREAMS of Decode (identical accept/reject
-decision and length for well-formed and malformed input alike)."""
-import numpy as np
-from hypothesis import given, settings, strategies as st
-
-import oracle
+"""Differential pinning of the oracle restatement against the reference's upstream C engine, CPU only:
+seeded samples of arbitrary byte strings as INPUT of Encode (identical bytes and return codes for every
+capacity class) and as COMPRESSED STREAMS of Decode (identical accept/reject decision and length for
+well-formed and malformed input alike), compared with that engine's recorded results
+(tests/golden/ref_engine.npz)."""
 from tests import inputs
 
-_P = oracle.Port()
-_R = oracle.Ref() if oracle.have_ref() else None
 
-_bytes = st.one_of(
-    st.binary(min_size=0, max_size=600),
-    st.builds(lambda b, k: (b * k)[:5000], st.binary(min_size=1, max_size=40), st.integers(1, 300)),
-    st.builds(lambda seed, n, hi: np.random.default_rng(seed).integers(0, hi, n, dtype=np.uint8).tobytes(),
-              st.integers(0, 2**31), st.integers(0, 3000), st.sampled_from([2, 4, 16, 256])),
-)
+def test_encode_port_equals_reference(port, ref):
+    ref.check("fuzz_encode", *inputs.fuzz_encode_rows(port, port))
 
 
-@settings(max_examples=250, deadline=None)
-@given(_bytes, st.integers(0, 40))
-def test_encode_port_equals_reference(data, slack):
-    if _R is None:
-        return
-    full = _R.encode(data)
-    assert _P.encode(data) == full
-    n = len(data)
-    for cap in {max(full[0] - slack, 1), n, 1024, full[0] + slack}:
-        if n == 0 or cap <= 0:
-            continue
-        assert _P.encode(data, cap) == _R.encode(data, cap)
-    if full[0] > 0:
-        assert _P.decode(full[1], n) == (n, data) if n else True
-
-
-@settings(max_examples=400, deadline=None)
-@given(st.binary(min_size=0, max_size=300), st.integers(0, 700))
-def test_decode_port_equals_reference_on_arbitrary_streams(stream, cap):
-    if _R is None:
-        return
-    a, b = _R.decode(stream, cap), _P.decode(stream, cap)
-    assert a[0] == b[0]
-    if a[0] > 0 and not inputs.uses_zero_offset(stream):   # offset-0 content is unspecified
-        assert a[1] == b[1]
+def test_decode_port_equals_reference_on_arbitrary_streams(port, ref):
+    ref.check("fuzz_decode", *inputs.fuzz_decode_rows(port, port))     # offset-0 content is unspecified
