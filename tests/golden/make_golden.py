@@ -18,8 +18,12 @@ orig/ holds the upstream lz4 C sources):
    tests/inputs.py -- encode, decode of malformed streams, dictionary and partial decode, XXH32, the
    data generator, and upstream lz4frame.c's frames -- which the tests compare the oracle and the
    frame writer with.  Needs libk4lz4.so built (the synth inputs), no GPU.
+4. hc_blocks.npz: blocks written by upstream LZ4_compress_HC (orig/lib/lz4hc.c) at levels 3, 9 and 12 --
+   fewer literals, longer matches and larger offsets than the fast encoder writes -- with the
+   (kind, size, seed, level) and CRC-32 of their raw data, which tests regenerate (inputs.hc_raw).
 """
 import base64
+import ctypes
 import hashlib
 import json
 import os
@@ -98,6 +102,26 @@ def main(ref_dir):
     sets["frame"] = np.array(inputs.frame_rows(P, upstream_frame)[1], dtype=np.int64)
     np.savez_compressed(inputs.REF_RESULTS, **sets)
     print({k: len(v) for k, v in sets.items()}, "reference results")
+
+    # 4. HC blocks
+    hc = R._lib.LZ4_compress_HC
+    hc.restype = ctypes.c_int
+    hc.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+    cols = {k: [] for k in ("kind", "size", "seed", "level", "crc")}
+    streams = []
+    for kind, size, seed in inputs.HC_INPUTS:
+        raw = np.frombuffer(inputs.hc_raw(P, kind, size, seed), dtype=np.uint8)
+        for level in (3, 9, 12):
+            dst = np.zeros(size + size // 255 + 16, dtype=np.uint8)
+            r = hc(raw.ctypes.data, dst.ctypes.data, size, dst.size, level)
+            assert r > 0 and P.decode(dst[:r], size) == (size, raw.tobytes()), (kind, size, level)
+            streams.append(dst[:r])
+            for k, v in zip(cols, (kind, size, seed, level, zlib.crc32(raw))):
+                cols[k].append(v)
+    off = np.concatenate([[0], np.cumsum([len(s) for s in streams])])
+    np.savez_compressed(inputs.HC_BLOCKS, streams=np.concatenate(streams), stream_off=off.astype(np.int64),
+                        **{k: np.array(v, dtype=None if k == "kind" else np.int64) for k, v in cols.items()})
+    print(len(streams), "HC blocks,", os.path.getsize(inputs.HC_BLOCKS), "bytes")
 
 
 if __name__ == "__main__":

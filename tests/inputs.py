@@ -306,6 +306,34 @@ def fuzz_decode_rows(port, eng, count: int = 1200):
     return labels, rows
 
 
+# ---- blocks written by upstream LZ4_compress_HC (golden/hc_blocks.npz) ------------------------------
+
+HC_BLOCKS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "hc_blocks.npz")
+HC_INPUTS = [(kind, size, seed) for seed, (kind, size) in enumerate(
+    [(k, n) for k in ("text2", "lowent", "runs", "datagen63") for n in (65536, 5000, 300, 40)], start=101)]
+
+
+def hc_raw(port, kind: str, size: int, seed: int) -> bytes:
+    """The raw data of an HC block: `gen`, or the reference data generator at match probability 0.63."""
+    if kind == "datagen63":
+        return port.datagen(size, 0.63, 0.0, seed).tobytes()
+    return gen(kind, size, seed)
+
+
+def hc_blocks(port):
+    """-> [(kind, size, level, stream, raw)] of golden/hc_blocks.npz, raw data regenerated and CRC-checked."""
+    with np.load(HC_BLOCKS) as z:
+        f = {k: z[k] for k in z.files}
+    out = []
+    for i in range(len(f["kind"])):
+        kind, size, seed = str(f["kind"][i]), int(f["size"][i]), int(f["seed"][i])
+        raw = hc_raw(port, kind, size, seed)
+        assert zlib.crc32(raw) == int(f["crc"][i]), (kind, size, seed)
+        stream = f["streams"][f["stream_off"][i]:f["stream_off"][i + 1]].tobytes()
+        out.append((kind, size, int(f["level"][i]), stream, raw))
+    return out
+
+
 # every set above that an engine computes alone, by the name its results are stored under
 ENGINE_SETS = {"corpus": corpus_rows, "malformed": malformed_rows, "dictionary": dictionary_rows,
                "partial": partial_rows, "datagen": datagen_rows, "xxh32": xxh32_rows,
