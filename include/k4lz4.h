@@ -226,6 +226,12 @@ K4LZ4_API int64_t k4lz4_launch_count(void);
  * Synchronises the device.  Diagnostics only (tests assert that clean data stays on the tile path). */
 K4LZ4_API int32_t k4lz4_decode_stats(int32_t device, uint64_t *out4, int32_t reset);
 
+/* Encoder path counters of `device` since the last reset, blocks of n > 0 the batched encoder ran:
+ * out3[0] encoded by the shared-memory-table warps, [1] by the global-table warps (both below
+ * 65 547 bytes), [2] by the u32-table engine (65 547 bytes and more, either warp kind).
+ * Synchronises the device.  Diagnostics only. */
+K4LZ4_API int32_t k4lz4_encode_stats(int32_t device, uint64_t *out3, int32_t reset);
+
 #ifdef __cplusplus
 }
 #endif

@@ -23,7 +23,7 @@ SYMBOLS = [
     "k4lz4_copy_blocks_device", "k4lz4_decode_stats",
     "k4lz4_decode_dict", "k4lz4_partial_decode", "k4lz4_decode_dict_batch", "k4lz4_partial_decode_batch",
     "k4lz4_pickle_writer_bound", "k4lz4_pickle_writer_batch", "k4lz4_encode_x32", "k4lz4_encode_batch_x32",
-    "k4lz4_xxh32", "k4lz4_xxh32_batch",
+    "k4lz4_xxh32", "k4lz4_xxh32_batch", "k4lz4_encode_stats",
 ]
 
 
@@ -74,6 +74,7 @@ def lib():
     L.k4lz4_copy_blocks_device.argtypes = [vp, vp, vp, vp, vp, i32, vp, i32]
     L.k4lz4_copy_blocks_device.restype = i32
     L.k4lz4_decode_stats.argtypes = [i32, vp, i32]; L.k4lz4_decode_stats.restype = i32
+    L.k4lz4_encode_stats.argtypes = [i32, vp, i32]; L.k4lz4_encode_stats.restype = i32
     L.k4lz4_decode_dict.argtypes = [vp, i32, vp, i32, vp, i32]; L.k4lz4_decode_dict.restype = i32
     L.k4lz4_partial_decode.argtypes = [vp, i32, vp, i32]; L.k4lz4_partial_decode.restype = i32
     L.k4lz4_decode_dict_batch.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, i32]

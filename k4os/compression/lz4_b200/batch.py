@@ -235,6 +235,13 @@ def decode_stats(device: int = 0, reset: bool = False) -> dict:
     return {"tile": int(v[0]), "tile_big": int(v[1]), "generic": int(v[2]), "repair_walks": int(v[3])}
 
 
+def encode_stats(device: int = 0, reset: bool = False) -> dict:
+    """Encoder path counters (k4lz4_encode_stats): which warps encoded how many blocks."""
+    v = (C.c_uint64 * 3)()
+    N.check(N.lib().k4lz4_encode_stats(device, C.addressof(v), int(reset)))
+    return {"shared": int(v[0]), "global": int(v[1]), "u32": int(v[2])}
+
+
 def decode_dict_batch_host(blocks: Sequence, caps: Sequence[int], dicts: Sequence, device: int = 0):
     """LZ4Codec.Decode(source, target, dictionary) over a batch (k4lz4_decode_dict_batch, host memory).
     Returns (list of bytes, int32 results)."""

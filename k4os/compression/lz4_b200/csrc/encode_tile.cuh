@@ -282,6 +282,11 @@ __device__ int encode_spec_warp(const uint8_t* __restrict__ src, const uint8_t* 
 #undef RD8
 }
 
+// Encoder path counters (k4lz4_encode_stats): blocks of n > 0 encoded by [0] the shared-memory-table warps,
+// [1] the global-table warps (both with encode_spec_warp), [2] the u32-table engine (encode_block_warp, either
+// warp kind).  Diagnostics only: the tests read them to see which warps did the work.
+__device__ unsigned long long g_encode_stats[3];
+
 // Persistent encoder, one warp per block at a time, one warp per CTA (a CTA leaves as soon as ITS warp
 // runs out of blocks, so the CTAs of the next launch on another stream move in without a gap).  Blocks
 // are handed out by a device counter.  Input and output stay in global memory.  Two kernels pull from
@@ -316,7 +321,10 @@ __device__ __forceinline__ void encode_persistent_warp(
         int r;
         if (n_ >= LIMIT_64K) r = encode_block_warp(src, n_, dst, cap, 0x7fffffff, table, enforce32);
         else r = encode_spec_warp<false, false, GTAB, GTAB ? ENC_GTAG : (K4_ENC_TAGS ? 1 : 0)>(src, nullptr, (uint32_t)n_, dst, cap, 0x7fffffff, table);
-        if (lane == 0) outLen[b] = r <= 0 ? -1 : r;
+        if (lane == 0) {
+            outLen[b] = r <= 0 ? -1 : r;
+            atomicAdd(&g_encode_stats[n_ >= LIMIT_64K ? 2 : (GTAB ? 1 : 0)], 1ull);
+        }
         __syncwarp();
     }
 }

@@ -795,6 +795,19 @@ int32_t k4lz4_decode_stats(int32_t device, uint64_t* out4, int32_t reset) {
     return K4LZ4_OK;
 }
 
+int32_t k4lz4_encode_stats(int32_t device, uint64_t* out3, int32_t reset) {
+    if (device_count_cached() <= 0) return fail(K4LZ4_E_NODEVICE, "no CUDA device available");
+    if (!out3) return fail(K4LZ4_E_ARG, "null pointer argument");
+    DeviceGuard g(device);
+    if (!g.ok) return fail(K4LZ4_E_CUDA, "cudaSetDevice(%d) failed", device);
+    unsigned long long v[3] = {0, 0, 0};
+    CU_TRY(cudaDeviceSynchronize());
+    CU_TRY(cudaMemcpyFromSymbol(v, k4::g_encode_stats, sizeof(v)));
+    for (int i = 0; i < 3; i++) out3[i] = v[i];
+    if (reset) { unsigned long long z[3] = {0, 0, 0}; CU_TRY(cudaMemcpyToSymbol(k4::g_encode_stats, z, sizeof(z))); }
+    return K4LZ4_OK;
+}
+
 #ifdef K4_DT_PROFILE
 // tools-only build: per-phase cycle sums of the tile decoder (scratch/, never shipped)
 __attribute__((visibility("default"))) int32_t k4lz4_debug_prof(uint64_t* out32, int32_t reset) {
